@@ -26,6 +26,9 @@ A "step" is one pass of the hot path over one batch of FRAMES distinct synthetic
            frames (first / middle / last of the batch) against the CPU oracle, the checker.
 
 `--impl reference` times that CPU encoder alone (all host threads, one frame per thread).
+
+`--dump-outputs DIR` writes what the last timed step of `value` returned (see dump_outputs), so two
+builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -287,6 +290,36 @@ class Env:
         e1.record(self.stream)
         self.barrier()
         return self.reduce_max([e0.elapsed_time(e1)])[0] / steps
+
+
+DUMP_SAMPLE_BYTES = 15 << 20   # 60 MiB as float32: the whole dump stays under 64 MB
+DUMP_SEED = 2160
+
+
+def dump_sample_positions(total: int) -> np.ndarray:
+    """Sorted positions into the concatenation of every frame's scan bytes: all of them when they fit
+    DUMP_SAMPLE_BYTES, else one position drawn with DUMP_SEED from each of DUMP_SAMPLE_BYTES equal strata
+    (so the sample depends on `total` alone)."""
+    n = DUMP_SAMPLE_BYTES
+    if total <= n:
+        return np.arange(total, dtype=np.int64)
+    lo = np.arange(n + 1, dtype=np.int64) * total // n
+    return lo[:-1] + (np.random.default_rng(DUMP_SEED).random(n) * (lo[1:] - lo[:-1])).astype(np.int64)
+
+
+def dump_outputs(out_dir: str, torch, d_scan, d_len, d_ovf) -> None:
+    """What pixo_b200_jpeg_encode_dev hands its caller, as float .npy files: scan_lengths and
+    scan_overflow (one value per frame) and scan_bytes_sample, the bytes at dump_sample_positions of the
+    frames' scan bytes laid end to end in frame order (one step's scans are larger than the dump may be)."""
+    lens = d_len.cpu().numpy().astype(np.int64)
+    pos = dump_sample_positions(int(lens.sum()))
+    starts = np.cumsum(lens) - lens
+    frame = np.searchsorted(np.cumsum(lens), pos, side="right")
+    flat = torch.from_numpy(frame * d_scan.shape[1] + pos - starts[frame]).to(d_scan.device)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "scan_lengths.npy"), lens.astype(np.float64))
+    np.save(os.path.join(out_dir, "scan_overflow.npy"), d_ovf.cpu().numpy().astype(np.float64))
+    np.save(os.path.join(out_dir, "scan_bytes_sample.npy"), d_scan.reshape(-1)[flat].cpu().numpy().astype(np.float32))
 
 
 def sha(b) -> str:
@@ -601,6 +634,8 @@ def run_ours(args):
     enc_launches = ctx.launch_count - launches_enc0
     enc_ms = env.reduce_max([ev0.elapsed_time(ev1)])[0]
     scan_bytes = int(d_slen.sum())
+    if args.dump_outputs and rank == 0:   # every rank encodes the same frames
+        dump_outputs(args.dump_outputs, torch, d_scan, d_slen, d_sovf)
 
     # ---- the dominant kernel alone (roofline) ----
     for _ in range(3):
@@ -764,7 +799,10 @@ def main():
     ap.add_argument("--configs", default="C3,C4,C5,P444", help="comma list of side configurations, or 'none'")
     ap.add_argument("--cfg-steps", type=int, default=8)
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:
